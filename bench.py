@@ -61,6 +61,21 @@ def model_class(variant):
             "original": P.OriginalSuDORMRF}[variant]
 METRIC = "mixtures_per_sec_forward_4s_8kHz_2src"
 UNIT = "mixtures/s"
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(out_dir, name, t):
+    """Writes the output `t` ([batch, ...]) as out_dir/<name>.npy in float32.  Above DUMP_LIMIT_BYTES only a fixed,
+    seeded sample of its batch rows (in batch order) is written, so runs with the same arguments write the same rows."""
+    import numpy as np
+    t = t.detach().float().cpu()
+    row_bytes = 4 * t[0].numel()
+    if t.numel() * 4 > DUMP_LIMIT_BYTES:
+        keep = max(1, DUMP_LIMIT_BYTES // row_bytes)
+        rows = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        t = t[rows]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
 
 
 def load_peaks():
@@ -224,14 +239,14 @@ def cpu_forward_rate(w, sample_B, steps, warmup, budget_s=None):
         t_start = time.perf_counter()
         for _ in range(steps):
             t0 = time.perf_counter()
-            O.forward(cfg, sd, x)
+            y = O.forward(cfg, sd, x)
             times.append(time.perf_counter() - t0)
             if budget_s is not None and time.perf_counter() - t_start > budget_s and len(times) >= 3:
                 break
     times.sort()
     med = times[len(times) // 2]
     return {"rate": sample_B / med, "sec_per_step": med, "done": len(times), "threads": torch.get_num_threads(),
-            "logical_cpus": logical, "physical_cores": physical, "best": sample_B / times[0]}
+            "logical_cpus": logical, "physical_cores": physical, "best": sample_B / times[0], "last_output": y}
 
 
 def run_reference(args, w, wl_name):
@@ -239,7 +254,9 @@ def run_reference(args, w, wl_name):
     if rank != 0:
         return
     sample_B = 1
-    r = cpu_forward_rate(w, sample_B, max(args.steps, 10), max(args.warmup, 1), budget_s=150.0)
+    r = cpu_forward_rate(w, sample_B, args.steps, max(args.warmup, 1))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "estimates", r["last_output"])
     line = {
         "impl": "reference", "metric": METRIC, "value": r["rate"], "unit": UNIT, "n_gpus": args.gpus,
         "steps": r["done"], "warmup": max(args.warmup, 1), "ms_per_step": r["sec_per_step"] * 1e3,
@@ -332,6 +349,8 @@ def run_b200(args, w, wl_name):
         wall = time.perf_counter() - wall0
         clocks = sampler.stop() if sampler else None
         dev_ms = sum(s.elapsed_time(e) for s, e in evs)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, "estimates", y)      # the last timed replay's separated sources
 
         # ---- end to end: pinned host mixtures in, pinned host estimates out, every step ----
         host_y = torch.empty(B, w["kw"]["num_sources"], T).pin_memory()
@@ -735,6 +754,9 @@ def main():
     ap.add_argument("--workload", default="improved_u16_512", choices=sorted(WORKLOADS))
     ap.add_argument("--batch", type=int, default=0, help="per-GPU batch (default: the workload's)")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the short runs of BASELINE configs 3 / 4 / 5")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's estimates as DIR/estimates.npy (float32; "
+                         f"a seeded sample of batch rows above {DUMP_LIMIT_BYTES >> 20} MiB)")
     args = ap.parse_args()
     w = WORKLOADS[args.workload]
     if args.impl == "reference":

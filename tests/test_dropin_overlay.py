@@ -4,7 +4,11 @@ whole-module pickle written against those paths loads (README.md:75 `torch.load(
 
 The import block under test is the reference's own: dnn/experiments/run_improved_sudormrf.py:23-29
 and utils/simple_whamr_evaluation.py:40-44 (minus the modules that need comet_ml / glob2 /
-speechbrain, which are not installed in this image)."""
+speechbrain).
+
+The reference checkout is stood in for by a tree with its package layout (regular packages with empty
+``__init__.py``), holding the modules that block imports, with placeholder contents: placeholders of the
+accelerated modules that the overlay has to hide, and of the other modules that it must leave visible."""
 import os
 import subprocess
 import sys
@@ -12,7 +16,36 @@ import sys
 import pytest
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REFERENCE = "/root/reference"
+
+_PLACEHOLDER_MODEL = "class {0}:\n    '''placeholder: the overlay must resolve this name to sudo_rm_rf_b200'''\n"
+STAND_IN = {
+    "sudo_rm_rf/__init__.py": "",
+    "sudo_rm_rf/dnn/__init__.py": "",
+    "sudo_rm_rf/dnn/losses/__init__.py": "",
+    "sudo_rm_rf/dnn/losses/sisdr.py": "class PermInvariantSISDR:\n    def __init__(self, **kwargs):\n        pass\n",
+    "sudo_rm_rf/dnn/losses/snr.py": "class PermInvariantSNRwithZeroRefs:\n    pass\n",
+    "sudo_rm_rf/dnn/models/__init__.py": "",
+    "sudo_rm_rf/dnn/models/improved_sudormrf.py": _PLACEHOLDER_MODEL.format("SuDORMRF"),
+    "sudo_rm_rf/dnn/models/groupcomm_sudormrf_v2.py": _PLACEHOLDER_MODEL.format("GroupCommSudoRmRf"),
+    "sudo_rm_rf/dnn/models/causal_improved_sudormrf_v3.py": _PLACEHOLDER_MODEL.format("CausalSuDORMRF"),
+    "sudo_rm_rf/dnn/models/sudormrf.py": _PLACEHOLDER_MODEL.format("SuDORMRF"),
+    "sudo_rm_rf/dnn/experiments/__init__.py": "",
+    "sudo_rm_rf/dnn/experiments/utils/__init__.py": "",
+    "sudo_rm_rf/dnn/experiments/utils/improved_cmd_args_parser_v2.py": "def get_args():\n    return None\n",
+    "sudo_rm_rf/dnn/experiments/utils/mixture_consistency.py": "def apply(pr_batch, input_mixture, mix_weights_type='uniform'):\n"
+                                                                "    raise AssertionError('placeholder')\n",
+}
+
+
+@pytest.fixture(scope="module")
+def reference(tmp_path_factory):
+    """Root of a stand-in for the reference checkout."""
+    root = tmp_path_factory.mktemp("reference")
+    for rel, text in STAND_IN.items():
+        path = root / rel
+        path.parent.mkdir(parents=True, exist_ok=True)
+        path.write_text(text)
+    return str(root)
 
 PICKLE = r"""
 import io, sys, torch
@@ -69,36 +102,33 @@ print("runner imports ok")
 """
 
 
-def _run(script):
-    out = subprocess.run([sys.executable, "-c", script], capture_output=True, text=True, cwd="/tmp")
+def _run(script, cwd):
+    out = subprocess.run([sys.executable, "-c", script], capture_output=True, text=True, cwd=cwd)
     assert out.returncode == 0, out.stderr[-3000:]
     return out.stdout
 
 
-def test_overlay_import_paths_and_pickle():
-    assert "overlay ok" in _run(PICKLE.format(repo=REPO))
+def test_overlay_import_paths_and_pickle(tmp_path):
+    assert "overlay ok" in _run(PICKLE.format(repo=REPO), tmp_path)
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference checkout not present (GPU box)")
-def test_overlay_keeps_rest_of_reference_importable():
+def test_overlay_keeps_rest_of_reference_importable(reference, tmp_path):
     setup = (f"sys.path.insert(0, {REPO!r}); sys.path.insert(0, {REPO!r} + '/sudo_rm_rf_b200/dropin')\n"
-             f"sys.path.append({REFERENCE!r})")
-    assert "runner imports ok" in _run(RUNNER_IMPORTS.format(setup=setup, reference=REFERENCE))
+             f"sys.path.append({reference!r})")
+    assert "runner imports ok" in _run(RUNNER_IMPORTS.format(setup=setup, reference=reference), tmp_path)
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference checkout not present (GPU box)")
-def test_meta_path_redirect_with_reference_first():
+def test_meta_path_redirect_with_reference_first(reference, tmp_path):
     """`sudo_rm_rf_b200.dropin.install()`: reference FIRST on sys.path, only the accelerated names are redirected."""
-    setup = (f"sys.path.insert(0, {REPO!r}); sys.path.insert(0, {REFERENCE!r})\n"
+    setup = (f"sys.path.insert(0, {REPO!r}); sys.path.insert(0, {reference!r})\n"
              "import sudo_rm_rf_b200.dropin as D; D.install()")
-    assert "runner imports ok" in _run(RUNNER_IMPORTS.format(setup=setup, reference=REFERENCE))
+    assert "runner imports ok" in _run(RUNNER_IMPORTS.format(setup=setup, reference=reference), tmp_path)
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference checkout not present (GPU box)")
-def test_overlay_without_reference_modules_fails_normally():
+def test_overlay_without_reference_modules_fails_normally(reference, tmp_path):
     """A module neither the overlay nor the reference has is a plain ModuleNotFoundError."""
     script = (f"import sys; sys.path.insert(0, {REPO!r}); sys.path.insert(0, {REPO!r} + '/sudo_rm_rf_b200/dropin')\n"
-              f"sys.path.append({REFERENCE!r})\n"
+              f"sys.path.append({reference!r})\n"
               "try:\n    import sudo_rm_rf.dnn.models.no_such_model\n"
               "except ModuleNotFoundError:\n    print('fine')\n")
-    assert "fine" in _run(script)
+    assert "fine" in _run(script, tmp_path)

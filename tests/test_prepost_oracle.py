@@ -65,20 +65,23 @@ def test_pit_sisdr_matches_reference_golden(ci):
     assert torch.allclose(-best.mean(), t["loss"][0], atol=1e-4, rtol=0)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/sudo_rm_rf"), reason="reference tree not present")
-def test_pit_sisdr_live_against_reference():
-    import sys
-    import warnings
-    sys.path.insert(0, "/root/reference")
-    warnings.filterwarnings("ignore")
-    import sudo_rm_rf.dnn.losses.sisdr as ref
+def pit_live_inputs():
+    """Seeded (estimates, targets, mixtures): 6 items, 3 sources, estimates a permutation of the targets + noise."""
     g = torch.Generator().manual_seed(5)
     tgt = torch.randn(6, 3, 3000, generator=g)
     est = tgt[:, [2, 0, 1]] + 0.3 * torch.randn(6, 3, 3000, generator=g)
     mix = tgt.sum(1, keepdim=True)
-    fn = ref.PermInvariantSISDR(batch_size=6, zero_mean=True, n_sources=3, backward_loss=False,
-                                improvement=True, return_individual_results=True)
-    want, perms = fn(est, tgt, initial_mixtures=mix, return_best_permutation=True)
+    return est, tgt, mix
+
+
+def test_pit_sisdr_live_against_reference():
+    """The reference's PermInvariantSISDR(zero_mean, improvement, return_best_permutation) on these seeded inputs,
+    stored by golden/make_golden_reference.py."""
+    est, tgt, mix = pit_live_inputs()
+    z = np.load(os.path.join(GOLDEN_DIR, "reference_sisdr.npz"))
+    np.testing.assert_allclose([float(est.double().sum()), float(tgt.double().sum())], z["pit_live/fingerprint"],
+                               rtol=1e-12)
+    want, perms = torch.from_numpy(z["pit_live/best"]), z["pit_live/perms"]
     best, idx = O.pit_sisdr(est, tgt, mix, zero_mean=True, improvement=True)
     assert torch.allclose(best, want, atol=1e-5, rtol=0)
     allp = list(itertools.permutations(range(3)))
